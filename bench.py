@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the DDPO hot path on B200 (contract: see the task brief / DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--phase sample|ppo]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--phase sample|ppo] [--dump-outputs DIR]
 
 Workload = BASELINE.json configs[1]: DDPO, SD2-base 512 px (64x64x4 latents, 77x1024 context), 50-step
 DDIM, CFG 5.0, eta 1.0, per-GPU sample batch 8 (global batch 64 on 8 GPUs), synthetic latents/prompt
@@ -20,6 +20,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -35,6 +36,14 @@ TRAIN_MACRO = int(os.environ.get("DDPO_BENCH_MACRO", "25"))  # timesteps of the 
 GUIDANCE, ETA, CLIP = 5.0, 1.0, 1e-4
 UNET_GFLOP = 804.3  # algorithmic GFLOP of one SD2-base U-Net application (SURVEY.md §8d / BASELINE.md §2)
 WORKLOAD = "DDPO SD2-base 512px, 50-step DDIM, CFG 5.0, eta 1.0, sample batch 8/GPU (BASELINE configs[1])"
+GRAD_SAMPLE = 1 << 20  # gradient entries --dump-outputs keeps (4 MB; the whole fp32 gradient is 3.5 GB)
+
+
+def _write_outputs(path, arrays):
+    """--dump-outputs: one float32 .npy per array, so that two builds can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def _peaks():
@@ -305,7 +314,14 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: 8 samples per GPU per epoch (default); strong: 64 samples per epoch for the whole job "
                          "(SURVEY 8d: sample batch 8 x 8/N batches per GPU), visible in the epoch-driver e2e number")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of each phase returned as DIR/<name>.npy "
+                         "(float32; rank 0): sample_next_latents, sample_log_probs, ppo_loss, ppo_approx_kl, ppo_clipfrac "
+                         "and ppo_grad_sample, the accumulated U-Net gradient at %d fixed indices (numpy default_rng(0))"
+                         % GRAD_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -382,6 +398,10 @@ def main():
         step(i)
     e1.record()
     torch.cuda.synchronize()
+    outputs = {}   # what the last timed step of each phase returned, for --dump-outputs
+    if args.dump_outputs:
+        outputs["sample_next_latents"] = S["x_next"].view(B, 4, 64, 64).cpu().numpy()
+        outputs["sample_log_probs"] = S["logp"].cpu().numpy()
     if world > 1:
         dist.barrier()
     ms = e0.elapsed_time(e1)
@@ -546,9 +566,15 @@ def main():
         t0e, t1e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t0e.record()
         for i in range(args.steps):
-            pg.train_step(tstate, batches[i % len(batches)], st, sched, True, GUIDANCE, ETA, CLIP, False, micro_batch_size=Bt, pmean_info=False)
+            _, last_info = pg.train_step(tstate, batches[i % len(batches)], st, sched, True, GUIDANCE, ETA, CLIP, False,
+                                         micro_batch_size=Bt, pmean_info=False)
         t1e.record()
         torch.cuda.synchronize()
+        if args.dump_outputs:
+            for k, v in last_info.items():
+                outputs[f"ppo_{k}"] = v.cpu().numpy().reshape(1)
+            idx = np.random.default_rng(0).integers(0, tstate.grad_acc.numel(), GRAD_SAMPLE)
+            outputs["ppo_grad_sample"] = tstate.grad_acc[torch.from_numpy(idx).to(dev)].cpu().numpy()
         if world > 1:
             dist.barrier()
         tt = torch.tensor([t0e.elapsed_time(t1e)], device=dev)
@@ -648,7 +674,9 @@ def main():
             argv = ["--dataset", "compressed_animals", "--sample_batch_size", str(B), "--num_sample_batches_per_epoch", str(nsb),
                     "--train_batch_size", str(TRAIN_BATCH), "--train_macro", str(TRAIN_MACRO), "--num_train_epochs", "3",
                     "--save_freq", "1000000", "--savepath", f"bench_driver_{rank}", "--seed", "0"]
-            with contextlib.redirect_stdout(sys.stderr):
+            # the driver writes its logs/ (args, sample images, rewards) under the working directory: a temporary one, so
+            # that the benchmark leaves the source tree untouched and runs from a read-only one
+            with tempfile.TemporaryDirectory() as tmp, contextlib.chdir(tmp), contextlib.redirect_stdout(sys.stderr):
                 out = PG.main(argv, models=(pipe, {"unet": net.params, "scheduler": state, "text_encoder": {}}),
                               max_epochs=3, save_last=False)
             # epoch 0 warms up (graph capture, arena growth); of the two steady-state epochs the faster one is reported
@@ -755,6 +783,8 @@ def main():
                                    "+ 1 optimizer update per 2 samples; a step = one denoising step or one train pass",
                            "samples_per_epoch_per_gpu": nb_}
         line["gpu_mem_peak_gb"] = round(torch.cuda.max_memory_allocated() / 2 ** 30, 2)
+        if args.dump_outputs:
+            _write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     # orderly teardown: drop captured graphs and cached buffers before the process exits
     torch.cuda.synchronize()

@@ -28,6 +28,9 @@ def emulated(monkeypatch, tmp_path):
     monkeypatch.setattr(V, "Arena", E.CpuArena)
     monkeypatch.setattr(PG, "USE_CUDA_GRAPH", False)
     monkeypatch.setattr(RWR, "USE_CUDA_GRAPH", False)
+    # the drivers put their own tensors (scheduler tables, epoch buffers) on the GPU whenever one exists; hide it so that
+    # they take the same host path on a machine with a GPU as on one without
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)
     PG._GRAPHS.clear()
     RWR._GRAPHS.clear()
     monkeypatch.chdir(tmp_path)
